@@ -20,9 +20,14 @@ so the genome is the survey's self-contained tier scaled to GRCh38: 24 chromosom
 repeat families, N blocks, ~27 k genes / ~350 k annotated junctions (tools/synth.py preset "grch38"), index
 (Genome 3.2 GB, SA 24 GB, SAindex 1.6 GB; --genomeSAindexNbases 14, --sjdbOverhang 99) built ONCE per box by this
 repository's own `--runMode genomeGenerate` on the GPU and cached under the work directory; both arms load that
-directory.  `--preset chr21` selects the 46.7 Mb genome of round 1 (index built by the reference's genomeGenerate).
+directory.  `--preset chr21` selects the 46.7 Mb genome of round 1 (index built by the reference's genomeGenerate when
+oracle/_ref/STAR was built, otherwise by this repository's, which writes the same files).
+
+--dump-outputs DIR writes the read results and alignment records of the last timed step of the value leg for a fixed, seeded
+sample of the reads (dump_outputs): the inputs depend only on the arguments, so two builds can be compared output for output.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--preset grch38|chr21] [--mm 0.005] [--read-len 100]
+                  [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...      (one rank per GPU; reads are sharded, weak scaling)
 """
 import argparse
@@ -37,6 +42,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the tree may be read-only: the modules imported from tools/ and tests/ leave no bytecode there
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 REF_STAR = os.path.join(ROOT, "oracle", "_ref", "STAR")
@@ -44,6 +50,8 @@ OUR_STAR = os.path.join(ROOT, "star_b200", "bin", "STAR")
 METRIC = "reads/sec (2x100 bp PE)"
 UNIT = "read pairs/s"
 SAINDEX_NBASES = {"tiny": 7, "small": 9, "chr21": 11, "grch38_8th": 13, "grch38": 14}
+DUMP_READS = 32768       # --dump-outputs: size of the fixed sample of reads
+DUMP_BYTES = 63 << 20    # and the most data it writes (with the .npy headers: < 64 MB)
 
 
 def log(*a):
@@ -79,8 +87,11 @@ def allowed_cpus():
     return n
 
 
-def prepare_genome(workdir, preset, device=0):
-    """genome.fa + annot.gtf + idx/ under workdir (built once, cached).  Returns (chrs, trs, idx_dir, build_info)."""
+def prepare_genome(workdir, preset, device=0, own_generate=False):
+    """genome.fa + annot.gtf + idx/ under workdir (built once, cached).  Returns (chrs, trs, idx_dir, build_info).
+
+    The index is built by the reference's generator for the small presets when oracle/_ref/STAR was built, otherwise by this repository's
+    GPU generator, which writes the same files (tests/test_gpu_config_gate.py checks them against the reference's digests)."""
     import synth
     t0 = time.time()
     chrs = synth.make_genome(preset)
@@ -95,7 +106,8 @@ def prepare_genome(workdir, preset, device=0):
         synth.write_fasta(chrs, os.path.join(workdir, "genome.fa"))
         synth.write_gtf(chrs, trs, os.path.join(workdir, "annot.gtf"))
         t_files = time.time() - t0
-        big = bool(synth.PRESETS[preset].get("big")) or os.environ.get("STAR_B200_BENCH_OWN_GENERATE") == "1"
+        big = (own_generate or bool(synth.PRESETS[preset].get("big")) or os.environ.get("STAR_B200_BENCH_OWN_GENERATE") == "1"
+               or not os.path.exists(REF_STAR))
         threads = str(min(64, os.cpu_count() or 8))
         args = ["--runMode", "genomeGenerate", "--genomeDir", "idx", "--genomeFastaFiles", "genome.fa", "--sjdbGTFfile", "annot.gtf",
                 "--sjdbOverhang", "99", "--genomeSAindexNbases", str(SAINDEX_NBASES[preset]), "--runThreadN", threads, "--outFileNamePrefix", "gen_"]
@@ -221,6 +233,29 @@ def cli_run(idx, fq1, fq2, out, threads, extra, device):
     return time.time() - t0
 
 
+def dump_outputs(path, res, al):
+    """--dump-outputs: what a caller of the timed path receives (the read results and their alignment records) for a fixed, seeded
+    sample of the reads, every field as <path>/result_<field>.npy and <path>/align_<field>.npy (float32 where that is exact, float64
+    otherwise; records in read order), and the sampled read indices as <path>/sample_reads.npy.  The sample is cut short where the
+    records would take it past DUMP_BYTES."""
+    import star_b200 as sb
+    as_float = lambda x: x.astype(np.float32 if x.dtype.itemsize <= 2 else np.float64)
+    sample = np.sort(np.random.default_rng(20260917).choice(len(res), size=min(len(res), DUMP_READS), replace=False))
+    rec_bytes = sum(as_float(np.zeros(1, sb.capi.ALIGN_DTYPE)[f]).nbytes for f in sb.capi.ALIGN_DTYPE.names)
+    res_bytes = 8 * (len(sb.capi.RESULT_DTYPE.names) + 1)   # float64 fields + the index in sample_reads
+    n_tr = res["nTrOut"][sample].astype(np.int64)
+    sample = sample[np.cumsum(res_bytes + n_tr * rec_bytes) <= DUMP_BYTES]
+    r = res[sample]
+    recs = al[np.concatenate([np.arange(o, o + k, dtype=np.int64) for o, k in zip(r["trOffset"], r["nTrOut"])] + [np.zeros(0, np.int64)])]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "sample_reads.npy"), sample.astype(np.float64))
+    for f in sb.capi.RESULT_DTYPE.names:
+        np.save(os.path.join(path, "result_%s.npy" % f), as_float(r[f]))
+    for f in sb.capi.ALIGN_DTYPE.names:
+        np.save(os.path.join(path, "align_%s.npy" % f), as_float(recs[f]))
+    log("outputs of the last timed step: %d sampled reads, %d records -> %s" % (len(sample), len(recs), path))
+
+
 def sam_records(path):
     with open(path, "rb") as f:
         return [l for l in f.read().split(b"\n") if l and not l.startswith(b"@")]
@@ -245,7 +280,11 @@ def main():
     ap.add_argument("--no-cli", action="store_true", help="skip the command-line leg")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--workdir", default=os.environ.get("STAR_B200_BENCH_DIR", "/tmp/star_b200_bench"))
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (value leg) for a fixed sample of the reads as DIR/<name>.npy (rank 0)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -387,6 +426,8 @@ def main():
     sync_all()
     wall = time.perf_counter() - t0
     launches = lib.star_gpu_launch_count() - launches0
+    if a.dump_outputs and rank == 0:   # outside the timed region; the e2e leg below overwrites these buffers
+        dump_outputs(a.dump_outputs, *eng.download(n, out=(res_np, al_np, ab)))
     # ---- e2e: host buffers through star_gpu_map_chunk
     for _ in range(max(1, a.warmup // 2)):
         eng.map_chunk(seq_p, off_p, n, nm, out=(res_np, al_np, ab))

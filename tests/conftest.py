@@ -75,6 +75,41 @@ def twopass_golden(tmp_path_factory):
     return str(d / "twopass")
 
 
+def refcmp_key(group, *params):
+    """Key of one case in tests/golden/refcmp.json: the group and the case's parameters."""
+    import json
+    return group + " " + json.dumps(params, sort_keys=True)
+
+
+@pytest.fixture(scope="session")
+def refcmp():
+    """tests/golden/refcmp.json: summaries of outputs of the unmodified reference for the cases outside tiny.tar.gz (make_golden_refcmp.py).
+    refcmp(group, *params) is the entry of one case."""
+    import json
+    with open(os.path.join(ROOT, "tests", "golden", "refcmp.json")) as f:
+        table = json.load(f)
+
+    def case(group, *params):
+        k = refcmp_key(group, *params)
+        assert k in table, "no reference outputs for %s: regenerate tests/golden/refcmp.json with tests/golden/make_golden_refcmp.py" % k
+        return table[k]
+    return case
+
+
+def sha256_lines(lines):
+    import hashlib
+    return hashlib.sha256(b"\n".join(lines)).hexdigest()
+
+
+def run_summary(prefix):
+    """Aligned.out.sam (records: count + digest), SJ.out.tab (digest) and the Log.final.out counters of a run, as refcmp.json stores them"""
+    import hashlib
+    body = sam_body(prefix + "Aligned.out.sam")
+    return {"sam_records": len(body), "sam_sha256": sha256_lines(body),
+            "sj_out_tab_sha256": hashlib.sha256(open(prefix + "SJ.out.tab", "rb").read()).hexdigest(),
+            "log_counters": [list(kv) for kv in log_counters(prefix + "Log.final.out")]}
+
+
 def check_twopass_outputs(out, ref):
     """Everything the reference writes in a junction-insertion / 2-pass run: records, junctions, counters of both passes, the junction
     database and (by digest) the rebuilt Genome / SA / SAindex."""

@@ -16,7 +16,11 @@ ROOT = cf.ROOT
 
 def parse_bam(path):
     raw = open(path, "rb").read()
-    d = gzip.decompress(raw)
+    return (raw,) + parse_bam_stream(gzip.decompress(raw))
+
+
+def parse_bam_stream(d):
+    """header text, references and records of a decompressed BAM stream"""
     assert d[:4] == b"BAM\x01"
     lt = struct.unpack("<i", d[4:8])[0]
     text = d[8:8 + lt]
@@ -33,7 +37,7 @@ def parse_bam(path):
         bs = struct.unpack("<i", d[o:o + 4])[0]
         recs.append(d[o:o + 4 + bs])
         o += 4 + bs
-    return raw, text, refs, recs
+    return text, refs, recs
 
 
 def check_bgzf(raw):
@@ -54,6 +58,12 @@ def _header_lines(text):
     return [l for l in text.split(b"\n") if not l.startswith(b"@PG") and not l.startswith(b"@CO")]
 
 
+def bam_summary(text, refs, recs):
+    """header lines (without @PG / @CO), references, number and digest of the records: how refcmp.json stores a BAM file of the reference"""
+    return {"header": [l.decode() for l in _header_lines(text)], "refs": [[n.decode(), ln] for n, ln in refs], "records": len(recs),
+            "records_sha256": cf.sha256_lines(recs)}
+
+
 CASES = [
     ("std", []),
     ("hard", []),
@@ -64,25 +74,21 @@ CASES = [
 ]
 
 
-@pytest.mark.skipif(not os.path.exists(oc.REF_STAR), reason="oracle/_ref/STAR not built (needs /root/reference)")
+def input_files(golden, base):
+    return [os.path.join(golden, base + "_1.fq")] + ([os.path.join(golden, base + "_2.fq")] if base != "se" else [])
+
+
 @pytest.mark.parametrize("base,extra", CASES)
-def test_bam_records_equal_the_reference(oracle, golden, tmp_path, base, extra):
-    files = [os.path.join(golden, base + "_1.fq")] + ([os.path.join(golden, base + "_2.fq")] if base != "se" else [])
-    outs = {}
-    for tag, binary, thr in (("ref", oc.REF_STAR, 1), ("ora", oc.ORACLE_CLI, 3)):
-        out = str(tmp_path / tag) + "/"
-        os.makedirs(out)
-        cmd = [binary, "--genomeDir", os.path.join(golden, "idx"), "--readFilesIn"] + files + ["--outFileNamePrefix", out, "--runThreadN", str(thr),
-               "--outSAMtype", "BAM", "Unsorted"] + extra + (["--gpuChunkReads", "700"] if tag == "ora" else [])
-        subprocess.check_call(cmd, stdout=subprocess.DEVNULL, cwd=out)
-        assert not os.path.exists(out + "Aligned.out.sam")
-        outs[tag] = parse_bam(out + "Aligned.out.bam")
-    assert check_bgzf(outs["ora"][0]) >= 2
-    assert outs["ora"][2] == outs["ref"][2]
-    assert _header_lines(outs["ora"][1]) == _header_lines(outs["ref"][1])
-    assert len(outs["ora"][3]) == len(outs["ref"][3])
-    for k, (x, y) in enumerate(zip(outs["ora"][3], outs["ref"][3])):
-        assert x == y, "record %d differs" % k
+def test_bam_records_equal_the_reference(oracle, golden, refcmp, tmp_path, base, extra):
+    """Against the reference's file (refcmp.json, written by the reference with --runThreadN 1)."""
+    out = str(tmp_path) + "/"
+    cmd = [oc.ORACLE_CLI, "--genomeDir", os.path.join(golden, "idx"), "--readFilesIn"] + input_files(golden, base) + ["--outFileNamePrefix", out,
+           "--runThreadN", "3", "--outSAMtype", "BAM", "Unsorted"] + extra + ["--gpuChunkReads", "700"]
+    subprocess.check_call(cmd, stdout=subprocess.DEVNULL, cwd=out)
+    assert not os.path.exists(out + "Aligned.out.sam")
+    raw, text, refs, recs = parse_bam(out + "Aligned.out.bam")
+    assert check_bgzf(raw) >= 2
+    assert bam_summary(text, refs, recs) == refcmp("bam", base, extra)["bam"]
 
 
 def test_bam_record_count_and_names_match_the_sam_golden(oracle, golden, tmp_path):
@@ -147,29 +153,21 @@ SORT_CASES = [
 ]
 
 
-@pytest.mark.skipif(not os.path.exists(oc.REF_STAR), reason="oracle/_ref/STAR not built (needs /root/reference)")
 @pytest.mark.parametrize("base,extra", SORT_CASES)
-def test_sorted_bam_equals_the_reference(oracle, golden, tmp_path, base, extra):
+def test_sorted_bam_equals_the_reference(oracle, golden, refcmp, tmp_path, base, extra):
     """--outSAMtype BAM Unsorted SortedByCoordinate: both files; the sorted one must list the same records in the same order as the
-    reference's bin-sorted file (coordinate, then read order; unmapped reads last in read order), header with SO:coordinate."""
-    files = [os.path.join(golden, base + "_1.fq")] + ([os.path.join(golden, base + "_2.fq")] if base != "se" else [])
-    outs = {}
-    for tag, binary, thr in (("ref", oc.REF_STAR, 2), ("ora", oc.ORACLE_CLI, 3)):
-        out = str(tmp_path / tag) + "/"
-        os.makedirs(out)
-        cmd = [binary, "--genomeDir", os.path.join(golden, "idx"), "--readFilesIn"] + files + ["--outFileNamePrefix", out, "--runThreadN", str(thr),
-               "--outSAMtype", "BAM", "Unsorted", "SortedByCoordinate"] + extra + (["--gpuChunkReads", "500"] if tag == "ora" else [])
-        subprocess.check_call(cmd, stdout=subprocess.DEVNULL, cwd=out)
-        outs[tag] = (parse_bam(out + "Aligned.sortedByCoord.out.bam"), parse_bam(out + "Aligned.out.bam"))
-    srt_o, uns_o = outs["ora"]
-    srt_r, uns_r = outs["ref"]
+    reference's bin-sorted file (coordinate, then read order; unmapped reads last in read order), header with SO:coordinate.
+    Reference files: refcmp.json, written by the reference with --runThreadN 2."""
+    out = str(tmp_path) + "/"
+    cmd = [oc.ORACLE_CLI, "--genomeDir", os.path.join(golden, "idx"), "--readFilesIn"] + input_files(golden, base) + ["--outFileNamePrefix", out,
+           "--runThreadN", "3", "--outSAMtype", "BAM", "Unsorted", "SortedByCoordinate"] + extra + ["--gpuChunkReads", "500"]
+    subprocess.check_call(cmd, stdout=subprocess.DEVNULL, cwd=out)
+    ref = refcmp("sorted", base, extra)
+    srt_o, uns_o = parse_bam(out + "Aligned.sortedByCoord.out.bam"), parse_bam(out + "Aligned.out.bam")
     check_bgzf(srt_o[0])
     assert srt_o[1].startswith(b"@HD\tVN:1.4\tSO:coordinate\n")
-    assert _header_lines(srt_o[1]) == _header_lines(srt_r[1]) and srt_o[2] == srt_r[2]
-    assert len(srt_o[3]) == len(srt_r[3])
-    for k, (x, y) in enumerate(zip(srt_o[3], srt_r[3])):
-        assert x == y, "sorted record %d differs" % k
+    assert bam_summary(*srt_o[1:]) == ref["sorted"]
     # the unsorted file next to it is unchanged by the extra output (the reference runs 2 threads here: compare as a multiset)
-    assert sorted(uns_o[3]) == sorted(uns_r[3])
+    assert bam_summary(uns_o[1], uns_o[2], sorted(uns_o[3])) == ref["unsorted_as_multiset"]
     keys = [struct.unpack("<II", r[4:12]) for r in srt_o[3]]
     assert keys == sorted(keys), "not coordinate-sorted"

@@ -1,16 +1,18 @@
 """The bit-identity gate of BASELINE.json configs[0] at its real size, on the GPU (SURVEY.md §8(c), last bullet).
 
 Genome: the chr21-sized synthetic stand-in (46.7 Mb, 3 chromosomes, repeat families, N block, 1352 spliced transcripts -> sjdb; there is no
-real chr21 on the box), index built on the box by the UNMODIFIED reference's genomeGenerate.  The drop-in command line star_b200/bin/STAR
-(CUDA engine) and oracle/_ref/STAR --runThreadN 1 map the same FASTQ files; the SAM records, SJ.out.tab and the integer counters of
-Log.final.out must be byte-equal:
+real chr21 on the box), index built on the box by this repository's GPU genomeGenerate, whose files must equal the UNMODIFIED reference's
+(SHA-256 digests in tests/golden/gate_chr21.json, see make_golden_gate.py).  The drop-in command line star_b200/bin/STAR (CUDA engine) maps
+seeded FASTQ files; the SAM records, SJ.out.tab and the integer counters of Log.final.out must equal those of oracle/_ref/STAR
+--runThreadN 1 on the same files (record count + digests, counters as text, in the same JSON file):
   * 100 k pairs 2x100 at 0.5 % substitutions (configs[0]),
   * 20 k pairs 2x150 at 5 % substitutions (configs[2] shape: long recursion trees, pool / task caps, overflow tiers),
 and the engine's records for the same reads equal the oracle's field by field through the C-ABI.  The heavy tail that drives the
 design (windows with 35-45 seeds from the repeat families, tens of thousands of recursion nodes per read, bump pools with per-chunk
-offsets) only exists at this size.  Also here: this repository's GPU genomeGenerate reproduces the reference's index files of this genome.
+offsets) only exists at this size.  Also here: both suffix-sort paths of the GPU genomeGenerate reproduce the reference's index files.
 """
 import hashlib
+import json
 import os
 import subprocess
 
@@ -22,19 +24,32 @@ import conftest as cf
 pytestmark = pytest.mark.gpu
 
 ROOT = cf.ROOT
-REF = os.path.join(ROOT, "oracle", "_ref", "STAR")
 OURS = os.path.join(ROOT, "star_b200", "bin", "STAR")
+GOLDEN = os.path.join(ROOT, "tests", "golden", "gate_chr21.json")
+CASES = [("std100", 100_000, 100, 0.005), ("hard150", 20_000, 150, 0.05)]
+INDEX_FILES = ("Genome", "SA", "SAindex", "chrStart.txt", "chrLength.txt", "chrName.txt", "sjdbInfo.txt", "sjdbList.out.tab", "exonInfo.tab",
+               "transcriptInfo.tab")
 
 
 @pytest.fixture(scope="module")
 def chr21(tmp_path_factory):
-    """Work directory with genome.fa, annot.gtf and idx/ (reference genomeGenerate); shared with bench.py --preset chr21."""
+    """Work directory with genome.fa, annot.gtf and idx/ (this repository's genomeGenerate); shared with bench.py --preset chr21."""
     import bench
     import synth
     wd = os.path.join(os.environ.get("STAR_B200_BENCH_DIR", "/tmp/star_b200_bench"), "chr21")
     os.makedirs(wd, exist_ok=True)
-    chrs, trs, idx, _ = bench.prepare_genome(wd, "chr21")
-    return {"dir": wd, "chrs": chrs, "trs": trs, "idx": idx, "synth": synth}
+    chrs, trs, idx, _ = bench.prepare_genome(wd, "chr21", own_generate=True)
+    with open(GOLDEN) as f:
+        golden = json.load(f)
+    return {"dir": wd, "chrs": chrs, "trs": trs, "idx": idx, "synth": synth, "golden": golden}
+
+
+def digest(p):
+    h = hashlib.sha256()
+    with open(p, "rb") as f:
+        for blk in iter(lambda: f.read(1 << 24), b""):
+            h.update(blk)
+    return h.hexdigest()
 
 
 def _reads(c, n, read_len, mm, seed, tag):
@@ -51,21 +66,19 @@ def _run(binary, idx, f1, f2, out, extra=()):
     subprocess.check_call([binary, "--genomeDir", idx, "--readFilesIn", f1, f2, "--outFileNamePrefix", out + "/"] + list(extra), stdout=subprocess.DEVNULL, timeout=1500)
 
 
-@pytest.mark.parametrize("name,n,read_len,mm", [("std100", 100_000, 100, 0.005), ("hard150", 20_000, 150, 0.05)])
+@pytest.mark.parametrize("name,n,read_len,mm", CASES)
 def test_cli_equals_reference_at_config_size(lib, chr21, tmp_path, name, n, read_len, mm):
+    for f in INDEX_FILES:   # the outputs below are the reference's on its own index
+        assert digest(os.path.join(chr21["idx"], f)) == chr21["golden"]["index_sha256"][f], f
+    ref = chr21["golden"]["cases"][name]
     _, _, f1, f2 = _reads(chr21, n, read_len, mm, 77, "gate_" + name)
-    ours, ref = str(tmp_path / "ours"), str(tmp_path / "ref")
+    assert [digest(f) for f in (f1, f2)] == ref["reads_sha256"], "tools/synth.py no longer makes the reads the reference outputs belong to"
+    ours = str(tmp_path / "ours")
     _run(OURS, chr21["idx"], f1, f2, ours, ["--runThreadN", "16"])
-    _run(REF, chr21["idx"], f1, f2, ref, ["--runThreadN", "1"])
-    a, b = cf.sam_body(ours + "/Aligned.out.sam"), cf.sam_body(ref + "/Aligned.out.sam")
-    assert len(a) == len(b)
-    bad = [i for i in range(len(a)) if a[i] != b[i]]
-    assert not bad, "%d of %d SAM records differ, first:\n%s\n%s" % (len(bad), len(a), a[bad[0]], b[bad[0]])
-    assert open(ours + "/SJ.out.tab", "rb").read() == open(ref + "/SJ.out.tab", "rb").read()
-    assert cf.log_counters(ours + "/Log.final.out") == cf.log_counters(ref + "/Log.final.out")
+    assert cf.run_summary(ours + "/") == ref["outputs"]
 
 
-@pytest.mark.parametrize("name,n,read_len,mm", [("std100", 100_000, 100, 0.005), ("hard150", 20_000, 150, 0.05)])
+@pytest.mark.parametrize("name,n,read_len,mm", CASES)
 def test_engine_equals_oracle_at_config_size(lib, oracle, chr21, name, n, read_len, mm):
     """Through the C-ABI, one chunk: every field of every record, plus the work counters the roofline numerator is built from."""
     import oracle_capi as oc
@@ -91,19 +104,12 @@ def test_engine_equals_oracle_at_config_size(lib, oracle, chr21, name, n, read_l
 def test_gpu_generate_equals_reference_index_at_config_size(lib, chr21, tmp_path):
     """This repository's --runMode genomeGenerate (GPU suffix sort, both the 32-bit path and the batched 64-bit path that GRCh38 takes)
     writes the reference's Genome / SA / SAindex / junction files for the chr21-sized genome byte for byte."""
-    ref = chr21["idx"]
-
-    def digest(p):
-        h = hashlib.sha256()
-        with open(p, "rb") as f:
-            for blk in iter(lambda: f.read(1 << 24), b""):
-                h.update(blk)
-        return h.hexdigest()
+    ref = chr21["golden"]["index_sha256"]
     for tag, env in (("small_path", {}), ("large_path", {"STAR_B200_SA_LARGE_CAP": "30000000"})):
         out = str(tmp_path / tag)
         os.makedirs(out)
         subprocess.check_call([OURS, "--runMode", "genomeGenerate", "--genomeDir", out, "--genomeFastaFiles", os.path.join(chr21["dir"], "genome.fa"),
                                "--sjdbGTFfile", os.path.join(chr21["dir"], "annot.gtf"), "--sjdbOverhang", "99", "--genomeSAindexNbases", "11", "--runThreadN", "16",
                                "--outFileNamePrefix", out + "_log_"], stdout=subprocess.DEVNULL, env=dict(os.environ, **env), timeout=1500)
-        for f in ("Genome", "SA", "SAindex", "chrStart.txt", "chrLength.txt", "chrName.txt", "sjdbInfo.txt", "sjdbList.out.tab", "exonInfo.tab", "transcriptInfo.tab"):
-            assert digest(os.path.join(out, f)) == digest(os.path.join(ref, f)), (tag, f)
+        for f in INDEX_FILES:
+            assert digest(os.path.join(out, f)) == ref[f], (tag, f)
